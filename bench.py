@@ -25,6 +25,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # a benchmark run leaves the tree as it found it
 
 import numpy as np  # noqa: E402
 
@@ -320,7 +321,8 @@ class DeviceRun:
             self.dist.barrier()
         torch.cuda.synchronize()
 
-    def run(self, steps, warmup, local, rank):
+    def run(self, steps, warmup, local, rank, dump=None):
+        """dump: called with the last timed step's result (after the timed region) before it is freed."""
         import torch
         batch, w, cap, ctx = self.batch, self.w, self.cap, self.ctx
         for _ in range(warmup):
@@ -348,8 +350,55 @@ class DeviceRun:
         step_ms = ev0.elapsed_time(ev1) / steps
         info = last.info()  # raises on overflow / unsupported
         kern_ms = float(np.mean(ctx.kernel_times_ms(min(steps, 256))))
+        if dump is not None:
+            dump(last)
         last.free()
         return step_ms, kern_ms, int(info.selected_rows), int(launches), clocks
+
+
+DUMP_WINDOWS = 32          # --dump-outputs: seeded windows of consecutive result rows ...
+DUMP_WINDOW_ROWS = 2048    # ... of this many rows each (every row when fewer are selected)
+DUMP_LIMIT_BYTES = 32 << 20  # per workload: the headline and its cfg2 secondary stay within 64 MB together
+
+
+def dump_scan_result(res, w, out_dir, prefix):
+    """Writes what a caller of the timed scan receives, as float arrays two builds can compare exactly, into
+    out_dir/<prefix><name>.npy: selected_rows [1]; rows, the result row indices of the sample; per projected column i
+    proj<i>_null (0 / 1) and either proj<i> [rows, 2] float64 (high and low 32 bits of the value) or, for strings,
+    proj<i>_len and proj<i>_bytes (the sampled strings concatenated, one float32 per byte). A string cell comes back as an
+    address into the image, which differs from run to run, so the bytes it points at are written instead."""
+    n = int(res.selected_rows)
+    if n <= DUMP_WINDOWS * DUMP_WINDOW_ROWS:
+        windows = [(0, n)]
+    else:
+        picked = np.random.default_rng(0).choice(n // DUMP_WINDOW_ROWS, DUMP_WINDOWS, replace=False)
+        windows = [(int(s) * DUMP_WINDOW_ROWS, DUMP_WINDOW_ROWS) for s in np.sort(picked)]
+    out = {"selected_rows": np.array([n], dtype=np.float64),
+           "rows": np.concatenate([np.arange(s, s + k, dtype=np.float64) for s, k in windows])}
+    for i in range(len(w.proj)):
+        vals, nulls, lens, heaps = [], [], [], []
+        for s, k in windows:
+            data, aux, words = res.fetch_col(i, s, k)
+            r = np.arange(k)
+            nulls.append(((words[r // 64] >> (r % 64).astype(np.uint64)) & np.uint64(1)).astype(np.float32))
+            if w.proj_is_string[i]:
+                lens.append(aux.astype(np.float32))
+                heaps.append(res.fetch_strings(i, s, k)[0].astype(np.float32))
+            else:
+                v = data.astype(np.uint64)
+                vals.append(np.stack([(v >> np.uint64(32)).astype(np.float64), (v & np.uint64(0xffffffff)).astype(np.float64)], axis=1))
+        out[f"proj{i}_null"] = np.concatenate(nulls)
+        if w.proj_is_string[i]:
+            out[f"proj{i}_len"] = np.concatenate(lens)
+            out[f"proj{i}_bytes"] = np.concatenate(heaps)
+        else:
+            out[f"proj{i}"] = np.concatenate(vals)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes for {prefix} exceed {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), a)
 
 
 def e2e_run(local, table, w, rows_per_block, sel_hint, args, repeats, barrier, zero_copy=False):
@@ -396,7 +445,7 @@ def run_ours(args):
     if world > 1 and not dist.is_initialized():
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    if rank == 0:
+    if rank == 0 and os.access(ROOT, os.W_OK):   # a read-only tree is run as build() left it
         g.build()
     if world > 1:
         dist.barrier()
@@ -433,6 +482,11 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
         return t.tolist()
 
+    def dumper(name, w):
+        if not args.dump_outputs or rank != 0:
+            return None
+        return lambda res: dump_scan_result(res, w, args.dump_outputs, name + "_")
+
     # every rank pins its host buffers next to ITS GPU: report all of them, not rank 0's
     numa_all = [numa_node if numa_node is not None else -1]
     if world > 1:
@@ -462,7 +516,7 @@ def run_ours(args):
         batch = ctx.open_batch(table, device_image_ptr=d_image.data_ptr(), host_view=False, image_size=stride * tiles)
         cap = int(table.total_rows * 0.13)
         run = DeviceRun(ctx, stream, batch, w, cap, world, dist)
-        step_ms, kern_ms, selected, launches, clocks = run.run(args.steps, args.warmup, local, rank)
+        step_ms, kern_ms, selected, launches, clocks = run.run(args.steps, args.warmup, local, rank, dump=dumper("cfg3", w))
         batch.close()
         del d_image
         torch.cuda.empty_cache()
@@ -552,7 +606,7 @@ def run_ours(args):
         torch.cuda.synchronize()
         batch = ctx.open_batch(table, device_image_ptr=d_image.data_ptr())
         run = DeviceRun(ctx, stream, batch, w, int(table.total_rows * 0.30), world, dist)
-        step_ms, kern_ms, selected, launches, clocks = run.run(args.steps, args.warmup, local, rank)
+        step_ms, kern_ms, selected, launches, clocks = run.run(args.steps, args.warmup, local, rank, dump=dumper("cfg2", w))
         batch.close()
         e2e_ms, n_e2e, h2d, d2h, n_parts, e2e_steps, e2e_launches = e2e_run(local, table, w, 1400, 0.30, args, 1, barrier)
         assert n_e2e == selected
@@ -628,7 +682,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the cfg2 measurement")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the process to the GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed scan's results (rank 0's shard) to DIR/<workload>_<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "compaction"):
+        ap.error("--dump-outputs applies to the scan workloads of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.workload == "compaction":

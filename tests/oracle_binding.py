@@ -1,8 +1,11 @@
 """ctypes binding of the CPU oracle (oracle/libob_oracle.so). TEST INFRASTRUCTURE: only tests/,
 __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs import this."""
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -30,6 +33,9 @@ def _cpu_stamp():
 
 
 def build_oracle():
+    global ORACLE_LIB
+    if os.path.dirname(ORACLE_LIB) != ORACLE_DIR:   # already built for this host in a temporary directory
+        return ORACLE_LIB
     src = [os.path.join(ORACLE_DIR, f) for f in ("ob_oracle.c", "ob_stream_codecs.c", "ob_oracle.h", "Makefile")]
     stamp_file = os.path.join(ORACLE_DIR, ".built_on")
     stamp = _cpu_stamp()
@@ -40,7 +46,12 @@ def build_oracle():
         same_host = False
     stale = (not os.path.exists(ORACLE_LIB)) or not same_host or \
         any(os.path.getmtime(s) > os.path.getmtime(ORACLE_LIB) for s in src)
-    if stale:
+    if stale and not os.access(ORACLE_DIR, os.W_OK):   # read-only tree: this host's build goes to a temporary directory
+        out = tempfile.mkdtemp(prefix="ob_oracle_") + os.sep
+        atexit.register(shutil.rmtree, out, True)
+        subprocess.run(["make", "-B", "-C", ORACLE_DIR, "-s", "OUT=" + out, out + "libob_oracle.so"], check=True, capture_output=True)
+        ORACLE_LIB = out + "libob_oracle.so"
+    elif stale:
         subprocess.run(["make", "-B", "-C", ORACLE_DIR, "-s", "all"], check=True, capture_output=True)
         with open(stamp_file, "w") as f:
             f.write(stamp + "\n")

@@ -1,6 +1,8 @@
-"""The micro-block framing pinned to the REAL reference: ObMicroBlockHeader compiled from
-/root/reference/src/storage/blocksstable/ob_micro_block_header.cpp into oracle/_ref/libref_macro.so (with the real
-format_i32 / format_i64 of common/ob_record_header.h and the in-tree crc).
+"""The micro-block framing pinned to the REAL reference: ObMicroBlockHeader compiled from the reference's
+src/storage/blocksstable/ob_micro_block_header.cpp into oracle/_ref/libref_macro.so (with the real
+format_i32 / format_i64 of common/ob_record_header.h and the in-tree crc) when its sources are present. Without them the writer's
+blocks must be byte for byte the ones the reference accepted when tests/golden/writer_blocks.npz was made, and the oracle's
+verifier, which agrees with the reference on valid and corrupted blocks, stands in for the reference's check.
   * every block the writer emits -- every PAX codec, every CS column type, OBGPU_ENC_AUTO, NULL / NOP shapes -- must pass the
     reference's own ObMicroBlockHeader::deserialize_and_check_record (is_valid + header checksum + payload checksum);
   * the 64 header bytes must equal what the reference's init + set_header_checksum + serialize produce from the same facts;
@@ -16,14 +18,29 @@ import oracle_binding as ora
 
 
 def _ref():
+    """The live reference library, or None when it could not be built."""
     if not os.path.exists(ora.REF_MACRO_LIB):
-        pytest.skip("oracle/_ref/libref_macro.so not built (needs /root/reference)")
+        return None
     L = C.CDLL(ora.REF_MACRO_LIB)
     L.ref_micro_block_check.argtypes = [C.c_void_p, C.c_int64]
     L.ref_micro_header_build.restype = C.c_int64
     L.ref_micro_header_build.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_uint16, C.c_uint32, C.c_uint8, C.c_uint16, C.c_uint32, C.c_int32,
                                          C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_int64]
     return L
+
+
+def oracle_block_check(b):
+    try:
+        return ora.Block(b).verify_checksums()
+    except Exception:
+        return -1   # ora_block_init already refuses the header
+
+
+def block_check(L):
+    """check(block) -> 0 when valid: the reference's deserialize_and_check_record, or the oracle's verifier without it."""
+    if L is None:
+        return oracle_block_check
+    return lambda b: L.ref_micro_block_check(b.ctypes.data, b.size)
 
 
 def blocks():
@@ -63,10 +80,14 @@ def blocks():
 
 def test_reference_accepts_every_writer_block_and_header_bytes_match():
     L = _ref()
+    G = None if L is not None else np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "writer_blocks.npz"))
     for name, b in blocks():
         b = np.ascontiguousarray(b)
-        assert L.ref_micro_block_check(b.ctypes.data, b.size) == 0, name
         assert ora.Block(b).verify_checksums() == 0, name
+        if L is None:   # the bytes the reference accepted, header included
+            assert np.array_equal(b, G[f"block_{name}"]), name
+            continue
+        assert L.ref_micro_block_check(b.ctypes.data, b.size) == 0, name
         h = b[:64]
         f16 = lambda o: int(np.frombuffer(h[o:o + 2].tobytes(), dtype=np.uint16)[0])
         f32 = lambda o: int(np.frombuffer(h[o:o + 4].tobytes(), dtype=np.uint32)[0])
@@ -90,11 +111,8 @@ def test_reference_and_oracle_refuse_the_same_corruptions():
                 continue
             bad = b.copy()
             bad[at] ^= 0x04
-            r_ref = L.ref_micro_block_check(bad.ctypes.data, bad.size)
-            try:
-                r_ora = ora.Block(bad).verify_checksums()
-            except Exception:
-                r_ora = -1   # ora_block_init already refuses the header
+            r_ora = oracle_block_check(bad)
+            r_ref = L.ref_micro_block_check(bad.ctypes.data, bad.size) if L is not None else r_ora
             assert (r_ref != 0) == (r_ora != 0), (name, at, r_ref, r_ora)
             assert r_ref != 0, (name, at)
 
@@ -104,7 +122,7 @@ def test_reference_accepts_the_device_encoders_blocks():
     import torch
     import oceanbase_b200 as ob
     from oceanbase_b200 import capi, compaction
-    L = _ref()
+    check = block_check(_ref())
     ctx = ob.ScanContext(0)
     rng = np.random.default_rng(23)
     n = 5000
@@ -117,7 +135,7 @@ def test_reference_accepts_the_device_encoders_blocks():
     img, off, sz = enc.fetch()
     for b in range(len(off)):
         blk = np.ascontiguousarray(img[off[b]:off[b] + sz[b]])
-        assert L.ref_micro_block_check(blk.ctypes.data, blk.size) == 0, b
+        assert check(blk) == 0, b
     enc.free()
     ctx.close()
 
@@ -127,7 +145,7 @@ def test_reference_accepts_random_tables_over_every_codec():
     the writer cuts passes the reference's check. (38 954 blocks over 1 200 seeds were checked this way when the pin was added.)"""
     import oceanbase_b200 as ob
     import test_gpu_fuzz as F
-    L = _ref()
+    check = block_check(_ref())
     n_blocks = 0
     for seed in range(30_000, 30_030):
         _rng, _cs, n, rpb, cols, _meta = F.random_case(ob, seed)
@@ -141,6 +159,6 @@ def test_reference_accepts_random_tables_over_every_codec():
             continue
         for b in range(table.n_blocks):
             blk = np.ascontiguousarray(table.block(b))
-            assert L.ref_micro_block_check(blk.ctypes.data, blk.size) == 0, (seed, b)
+            assert check(blk) == 0, (seed, b)
             n_blocks += 1
     assert n_blocks > 100

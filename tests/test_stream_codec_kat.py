@@ -1,9 +1,10 @@
 """K13 pin: the oracle's integer stream decoders (oracle/ob_stream_codecs.c) against the REAL reference codec library
-(oracle/_ref/libref_codec.so, compiled from /root/reference/deps/oblib/src/lib/codec by oracle/Makefile).
+(oracle/_ref/libref_codec.so, compiled by oracle/Makefile from the reference's deps/oblib/src/lib/codec when its sources are present).
 
 Every codec x width decodes what the reference ENCODER produced and must equal both the input and the reference
 DECODER's output. Datasets follow unittest/storage/blocksstable/cs_encoding/test_integer_stream.cpp:459-829
-(all zero, min / max, monotone, negative deltas, long runs, random) plus exception-heavy PFOR blocks."""
+(all zero, min / max, monotone, negative deltas, long runs, random) plus exception-heavy PFOR blocks. Without the reference's
+sources the same checks run on the streams the reference encoder produced for tests/golden/ref_vectors.npz."""
 import ctypes as C
 import os
 
@@ -15,6 +16,7 @@ import oracle_binding as ora
 TYPES = {1: "RAW", 2: "DOUBLE_DELTA_ZIGZAG_RLE", 3: "DOUBLE_DELTA_ZIGZAG_PFOR", 4: "DELTA_ZIGZAG_RLE", 5: "DELTA_ZIGZAG_PFOR",
          6: "SIMD_FIXEDPFOR", 8: "XOR_FIXED_PFOR"}
 WIDTHS = {1: np.uint8, 2: np.uint16, 4: np.uint32, 8: np.uint64}
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_vectors.npz")
 
 
 def datasets(dt, rng):
@@ -42,8 +44,9 @@ def datasets(dt, rng):
 
 
 def _ref():
+    """The live reference codec library, or None when it could not be built."""
     if not os.path.exists(ora.REF_CODEC_LIB):
-        pytest.skip("oracle/_ref/libref_codec.so not built (needs /root/reference)")
+        return None
     L = C.CDLL(ora.REF_CODEC_LIB)
     L.ref_codec_encode.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
     L.ref_codec_decode.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint64)]
@@ -59,6 +62,24 @@ def ref_encode(L, t, a):
     return out[:ol.value].copy()
 
 
+def reference_streams(L, t, ub, seed):
+    """(dataset name, values, the reference encoder's bytes) of codec t at width ub: from the live library L, or the committed
+    golden streams when L is None."""
+    dt = WIDTHS[ub]
+    if L is not None:
+        for name, a in datasets(dt, np.random.default_rng(seed)):
+            a = np.ascontiguousarray(a)
+            yield name, a, ref_encode(L, t, a)
+        return
+    G = np.load(GOLDEN)
+    n_cases = 0
+    for (gt, gub, n, vpos, epos, elen) in G["codec_index"]:
+        if gt == t and gub == ub:
+            n_cases += 1
+            yield f"golden {n_cases}", G["codec_values"][vpos:vpos + n].astype(dt), G["codec_bytes"][epos:epos + elen]
+    assert n_cases > 0, (t, ub)
+
+
 @pytest.mark.parametrize("t", sorted(TYPES))
 @pytest.mark.parametrize("ub", sorted(WIDTHS))
 def test_oracle_decodes_reference_streams(t, ub):
@@ -66,15 +87,12 @@ def test_oracle_decodes_reference_streams(t, ub):
     O = ora.oracle()
     O.ora_int_stream_decode.argtypes = [C.c_int32, C.c_uint32, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.POINTER(C.c_int64)]
     dt = WIDTHS[ub]
-    rng = np.random.default_rng(1000 * t + ub)
-    for name, a in datasets(dt, rng):
-        a = np.ascontiguousarray(a)
-        enc = ref_encode(L, t, a)
-        # the real decoder first (sanity of the door itself)
-        want = np.zeros(a.size, dtype=dt)
-        used = C.c_uint64(0)
-        assert L.ref_codec_decode(t, ub, enc.ctypes.data, enc.size, a.size, want.ctypes.data, C.byref(used)) == 0
-        assert np.array_equal(want, a), (TYPES[t], ub, name, a.size)
+    for name, a, enc in reference_streams(L, t, ub, 1000 * t + ub):
+        used = C.c_uint64(enc.size)
+        if L is not None:   # the real decoder first (sanity of the door itself)
+            want = np.zeros(a.size, dtype=dt)
+            assert L.ref_codec_decode(t, ub, enc.ctypes.data, enc.size, a.size, want.ctypes.data, C.byref(used)) == 0
+            assert np.array_equal(want, a), (TYPES[t], ub, name, a.size)
         got = np.zeros(a.size, dtype=dt)
         cons = C.c_int64(0)
         padded = np.concatenate([enc, np.zeros(16, dtype=np.uint8)])     # decoders may not read past in_len
@@ -88,13 +106,8 @@ def test_oracle_decodes_reference_streams(t, ub):
 @pytest.mark.parametrize("ub", sorted(WIDTHS))
 def test_writer_encoders_are_byte_exact(t, ub):
     """The writer's stream encoders (oceanbase_b200/csrc/stream_codecs_host.h) produce the reference encoders' bytes."""
-    L = _ref()
     from oceanbase_b200.capi import lib
-    dt = WIDTHS[ub]
-    rng = np.random.default_rng(77 * t + ub)
-    for name, a in datasets(dt, rng):
-        a = np.ascontiguousarray(a)
-        want = ref_encode(L, t, a)
+    for name, a, want in reference_streams(_ref(), t, ub, 77 * t + ub):
         v64 = np.ascontiguousarray(a.astype(np.uint64))
         n = C.c_int64(0)
         out = np.zeros(a.size * ub * 2 + 4096, dtype=np.uint8)
