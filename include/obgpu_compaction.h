@@ -195,6 +195,22 @@ int obgpu_encode_columns(obgpu_ctx *ctx, const obgpu_encode_col *cols, int32_t n
  * column (a column group of a column-oriented merge is one call with the group's columns: ObWriteHelper::project). */
 int obgpu_merge_result_encode(obgpu_merge_result *res, const int32_t *result_cols, const int32_t *obj_types, int32_t n_cols,
                               int32_t rowkey_col_cnt, int64_t rows_per_block, int32_t align, obgpu_encoded **out);
+/* The same with a codec per column. encodings[i]: OBGPU_ENC_RAW / _DICT / _RLE / _CONST / _INTEGER_BASE_DIFF (forced) or
+ * OBGPU_ENC_AUTO (chosen per micro-block like obgpu_writer_encode_table's OBGPU_ENC_AUTO); encodings == NULL: every column RAW.
+ * Byte for byte the host writer's blocks for the same rows and encodings. A block the host writer would encode differently
+ * from the device reads size 0 and counts in n_host_blocks: RAW (forced or chosen) with var-stored cells, or a forced codec the
+ * host writer refuses for the block's data (CONST with more than 32 exceptions or more than 10 % of the rows, DICT / RLE on a
+ * column whose every cell is NULL); encode those blocks with the host writer and the same encodings.
+ * INTEGER_BASE_DIFF over a single value is written as RAW, as the host writer does.
+ * Call-level refusals: a string column -> OBGPU_NOT_SUPPORTED; an encoding outside the six -> OBGPU_INVALID_ARGUMENT; some
+ * column not RAW and rows_per_block > 4096 (the codec kernel's cap) -> OBGPU_NOT_SUPPORTED; some column not RAW and the largest
+ * block the requested codecs can write, plus the kernel's per-row scratch, does not fit one CTA's shared memory
+ * -> OBGPU_NOT_SUPPORTED. Every column RAW runs the RAW encoder of obgpu_encode_columns. */
+int obgpu_encode_columns_with(obgpu_ctx *ctx, const obgpu_encode_col *cols, const int32_t *encodings, int32_t n_cols,
+                              int32_t rowkey_col_cnt, int64_t total_rows, int64_t rows_per_block, int32_t align, obgpu_encoded **out);
+int obgpu_merge_result_encode_with(obgpu_merge_result *res, const int32_t *result_cols, const int32_t *obj_types,
+                                   const int32_t *encodings, int32_t n_cols, int32_t rowkey_col_cnt, int64_t rows_per_block,
+                                   int32_t align, obgpu_encoded **out);
 typedef struct obgpu_encoded_info {
   int64_t image_size;    /* bytes of the image (aligned block slots)          */
   int64_t total_rows;

@@ -13,7 +13,7 @@ INC = os.path.join(_HERE, "..", "include")
 LIB = os.path.join(CSRC, "libobgpu_scan.so")
 WRITER_LIB = os.path.join(CSRC, "libobgpu_writer.so")
 SOURCES = ["obgpu_scan.cu"]
-HEADERS = ["ob_format.h", "scan_device.cuh", "scan_small.cuh", "merge_kernels.cuh", "merge_exchange.cuh", "merge_streamed.cuh", "encode_kernels.cuh", "macro_blocks.cuh", "dict_ops.cuh", "cg_bitmap.cuh", "result_strings.cuh", "skip_index.cuh", "stream_codecs.cuh", "mat_codecs.cuh", "host_pipeline.h",
+HEADERS = ["ob_format.h", "scan_device.cuh", "scan_small.cuh", "merge_kernels.cuh", "merge_exchange.cuh", "merge_streamed.cuh", "encode_kernels.cuh", "encode_codecs.cuh", "macro_blocks.cuh", "dict_ops.cuh", "cg_bitmap.cuh", "result_strings.cuh", "skip_index.cuh", "stream_codecs.cuh", "mat_codecs.cuh", "host_pipeline.h",
            os.path.join(INC, "obgpu_scan.h"), os.path.join(INC, "obgpu_compaction.h"), os.path.join(INC, "obgpu_skip_index.h"), os.path.join(INC, "obgpu_pipeline.h")]
 WRITER_SOURCES = ["sstable_writer.cpp"]
 WRITER_HEADERS = ["ob_format.h", "stream_codecs_host.h", os.path.join(INC, "obgpu_writer.h"), os.path.join(INC, "obgpu_scan.h"),

@@ -234,6 +234,8 @@ def declared_signatures():
         "obgpu_batch_open_macro_blocks": (C.c_int, [vp, vp, i64, i64, i32, i32, P(vp), P(i32)]),
         "obgpu_encode_columns": (C.c_int, [vp, P(EncodeCol), i32, i32, i64, i64, i32, P(vp)]),
         "obgpu_merge_result_encode": (C.c_int, [vp, vp, vp, i32, i32, i64, i32, P(vp)]),
+        "obgpu_encode_columns_with": (C.c_int, [vp, P(EncodeCol), vp, i32, i32, i64, i64, i32, P(vp)]),
+        "obgpu_merge_result_encode_with": (C.c_int, [vp, vp, vp, vp, i32, i32, i64, i32, P(vp)]),
         "obgpu_encoded_get_info": (C.c_int, [vp, P(EncodedInfo)]),
         "obgpu_encoded_fetch": (C.c_int, [vp, vp, i64, vp, vp, i32]),
         "obgpu_encoded_device_image": (C.c_int, [vp, P(vp), P(vp), P(vp)]),

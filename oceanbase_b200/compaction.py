@@ -286,8 +286,9 @@ def write_merged_sstable(res: MergeResult, rows_per_block: int = 1400, payload_e
 
 # ---- phase B on the device: merged columns -> SSTable bytes + column checksums -------------------------------------------
 class Encoded:
-    """Device-encoded micro-blocks (obgpu_encoded): PAX blocks, every column RAW, byte for byte what the host writer
-    produces (ObMicroBlockEncoder::build_block with ObRawEncoder on every column)."""
+    """Device-encoded micro-blocks (obgpu_encoded): PAX blocks, byte for byte what the host writer produces for the same rows
+    and per-column encodings (ObMicroBlockEncoder::build_block; RAW on every column unless encodings were given). A block of
+    size 0 is left to the host writer (info().n_host_blocks counts them)."""
 
     def __init__(self, ctx, handle, n_cols, keep=None):
         self.ctx, self._h, self.n_cols, self._keep = ctx, handle, n_cols, keep
@@ -341,12 +342,34 @@ def _encode_cols(cols):
     return arr
 
 
-def encode_columns(ctx, cols, total_rows: int, rows_per_block: int, rowkey_cnt: int = 0, align: int = 128, keep=None) -> Encoded:
-    """cols: (device pointer of the int64 value images, device pointer of the NULL bytes or None, OBJ_* type, byte_packing_only)."""
+DEVICE_ENCODINGS = (capi.ENC_RAW, capi.ENC_DICT, capi.ENC_RLE, capi.ENC_CONST, capi.ENC_INTEGER_BASE_DIFF, capi.ENC_AUTO)
+
+
+def _encodings(encodings, n_cols) -> np.ndarray:
+    """encodings -> int32 array of n_cols codecs the device encoder takes (RAW / DICT / RLE / CONST / INTEGER_BASE_DIFF / AUTO)."""
+    enc = np.ascontiguousarray(encodings, dtype=np.int32)
+    if enc.shape != (n_cols,):
+        raise ValueError(f"encodings: {n_cols} values expected, got {enc.size}")
+    bad = [int(e) for e in enc if int(e) not in DEVICE_ENCODINGS]
+    if bad:
+        raise ValueError(f"encodings: {bad} not among the device encoder's codecs {DEVICE_ENCODINGS}")
+    return enc
+
+
+def encode_columns(ctx, cols, total_rows: int, rows_per_block: int, rowkey_cnt: int = 0, align: int = 128, keep=None,
+                   encodings: Optional[Sequence[int]] = None) -> Encoded:
+    """cols: (device pointer of the int64 value images, device pointer of the NULL bytes or None, OBJ_* type, byte_packing_only).
+    encodings: one ENC_RAW / ENC_DICT / ENC_RLE / ENC_CONST / ENC_INTEGER_BASE_DIFF / ENC_AUTO per column (None: every column RAW)."""
     h = C.c_void_p()
+    if encodings is not None:
+        enc = _encodings(encodings, len(cols))
     arr = _encode_cols(cols)
-    check(lib.obgpu_encode_columns(ctx._h, arr, len(cols), rowkey_cnt, total_rows, rows_per_block, align, C.byref(h)),
-          "obgpu_encode_columns", ctx._h)
+    if encodings is None:
+        check(lib.obgpu_encode_columns(ctx._h, arr, len(cols), rowkey_cnt, total_rows, rows_per_block, align, C.byref(h)),
+              "obgpu_encode_columns", ctx._h)
+    else:
+        check(lib.obgpu_encode_columns_with(ctx._h, arr, enc.ctypes.data, len(cols), rowkey_cnt, total_rows, rows_per_block, align,
+                                            C.byref(h)), "obgpu_encode_columns_with", ctx._h)
     return Encoded(ctx, h, len(cols), keep)
 
 
@@ -358,27 +381,35 @@ def column_checksums(ctx, cols, total_rows: int) -> np.ndarray:
 
 
 def encode_merge_result(res: MergeResult, result_cols: Sequence[int], obj_types: Sequence[int], rows_per_block: int,
-                        rowkey_cnt: int = 1, align: int = 128) -> Encoded:
-    """One column group of the merged stream (-1: the rowkey, -2 ...: further rowkey columns, >= 0 payload columns)."""
+                        rowkey_cnt: int = 1, align: int = 128, encodings: Optional[Sequence[int]] = None) -> Encoded:
+    """One column group of the merged stream (-1: the rowkey, -2 ...: further rowkey columns, >= 0 payload columns).
+    encodings: one codec per column as in encode_columns (None: every column RAW)."""
     rc = np.ascontiguousarray(result_cols, dtype=np.int32)
     ot = np.ascontiguousarray(obj_types, dtype=np.int32)
     h = C.c_void_p()
-    check(lib.obgpu_merge_result_encode(res._h, rc.ctypes.data, ot.ctypes.data, len(rc), rowkey_cnt, rows_per_block, align,
-                                        C.byref(h)), "obgpu_merge_result_encode", res.ctx._h)
+    if encodings is None:
+        check(lib.obgpu_merge_result_encode(res._h, rc.ctypes.data, ot.ctypes.data, len(rc), rowkey_cnt, rows_per_block, align,
+                                            C.byref(h)), "obgpu_merge_result_encode", res.ctx._h)
+    else:
+        enc = _encodings(encodings, len(rc))
+        check(lib.obgpu_merge_result_encode_with(res._h, rc.ctypes.data, ot.ctypes.data, enc.ctypes.data, len(rc), rowkey_cnt,
+                                                 rows_per_block, align, C.byref(h)), "obgpu_merge_result_encode_with", res.ctx._h)
     return Encoded(res.ctx, h, len(rc), res)
 
 
 def co_merge_write(res: MergeResult, column_groups: Sequence[Sequence[int]], obj_types: Dict[int, int], rows_per_block: int,
-                   align: int = 128) -> List[Encoded]:
+                   align: int = 128, encodings: Optional[Dict[int, int]] = None) -> List[Encoded]:
     """Column-oriented merge, writer side (ObCOMergeLogReplayer::replay_merge_log -> ObCOMergeWriter -> ObWriteHelper::project /
     append, column_store/ob_column_oriented_merger.cpp:722-745, ob_co_merge_writer.cpp:67-117): the merged stream is produced
     ONCE and replayed into the writer of every column group; here every group is one obgpu_merge_result_encode over the columns
-    the group projects. A group that holds the rowkey (-1 first) is written with rowkey_cnt 1, a pure column group with 0."""
+    the group projects. A group that holds the rowkey (-1 first) is written with rowkey_cnt 1, a pure column group with 0.
+    encodings: column -> codec (as encode_columns takes them; a column it does not name is RAW); None: every column RAW."""
     out = []
     for cg in column_groups:
         cg = list(cg)
         rk = 1 if cg and cg[0] == -1 else 0
-        out.append(encode_merge_result(res, cg, [obj_types[c] for c in cg], rows_per_block, rowkey_cnt=rk, align=align))
+        enc = None if encodings is None else [encodings.get(c, capi.ENC_RAW) for c in cg]
+        out.append(encode_merge_result(res, cg, [obj_types[c] for c in cg], rows_per_block, rowkey_cnt=rk, align=align, encodings=enc))
     return out
 
 

@@ -30,8 +30,8 @@ struct ColSpec {
   const int64_t *vals;
   const uint8_t *nulls;
   uint64_t store_mask;     // low type_store_size bytes (ColCtx::uval)
-  uint8_t obj_type, byte_only, datum_len, pad0;
-  uint32_t pad1;
+  uint8_t obj_type, byte_only, datum_len, enc;   // enc: OBGPU_ENC_* of the column (codec kernel only)
+  uint8_t sc, ts, pad[2];                          // store class (1 signed, 2 unsigned), type_store_size
 };
 
 struct Params {
@@ -90,33 +90,18 @@ struct ColLayout {
   uint8_t attr, size, bp, has_null;
 };
 
-template <bool CKSUM>
-__global__ void __launch_bounds__(kThreads) obgpu_encode_blocks_kernel(const __grid_constant__ Params p) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  uint32_t *img32 = reinterpret_cast<uint32_t *>(smem);                 // block image, p.slot_cap bytes
-  uint32_t *tab = reinterpret_cast<uint32_t *>(smem + p.slot_cap);      // 4 x 256 crc tables
-  // per column scratch behind the tables: [kWarps][n_cols] max, [kWarps][n_cols] NULL count, [n_cols] layout
-  unsigned long long *s_wmax = reinterpret_cast<unsigned long long *>(smem + p.slot_cap + 4096u);
-  uint32_t *s_wnull = reinterpret_cast<uint32_t *>(s_wmax + kWarps * p.n_cols);
-  ColLayout *s_lay = reinterpret_cast<ColLayout *>(s_wnull + kWarps * p.n_cols);
-  __shared__ uint32_t s_red[kWarps];
-  __shared__ int s_blk;
-  __shared__ uint32_t s_size, s_original, s_ext_bit, s_host;
-  __shared__ long long s_off;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-
-  if (tid == 0) s_blk = atomicAdd(p.ticket, 1);
-  // zero image (cells are OR-ed in; padding up to the aligned slot must be zero): before anything else, under the ticket's round trip
-  for (uint32_t i = (uint32_t)tid; i < p.slot_cap / 16u; i += kThreads) reinterpret_cast<uint4 *>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
-  // crc tables (slicing by 4): tab[k * 256 + i] = crc of byte i followed by k zero bytes
-  for (int i = tid; i < 256; i += kThreads) {
+// ---- pieces shared by the RAW kernel and the codec kernel (encode_codecs.cuh); NT: threads of the CTA -------------------------
+// crc tables (slicing by 4): tab[k * 256 + i] = crc of byte i followed by k zero bytes
+template <int NT>
+__device__ __forceinline__ void build_crc_tables(uint32_t *tab, int tid) {
+  for (int i = tid; i < 256; i += NT) {
     uint32_t c = (uint32_t)i;
 #pragma unroll
     for (int k = 0; k < 8; ++k) c = (c & 1u) ? kCrcPoly ^ (c >> 1) : c >> 1;
     tab[i] = c;
   }
   __syncthreads();
-  for (int i = tid; i < 256; i += kThreads) {
+  for (int i = tid; i < 256; i += NT) {
     uint32_t c = tab[i];
 #pragma unroll
     for (int k = 1; k < 4; ++k) {
@@ -124,13 +109,14 @@ __global__ void __launch_bounds__(kThreads) obgpu_encode_blocks_kernel(const __g
       tab[k * 256 + i] = c;
     }
   }
-  const int blk = s_blk;
-  const int64_t row0 = (int64_t)blk * p.rows_per_block;
-  const uint32_t nrows = (uint32_t)min(p.rows_per_block, p.total_rows - row0);
-  const int nc = p.n_cols;
-  __syncthreads();
+}
 
-  // ---- stats (+ column checksums): four columns at a time, their loads in flight together ---------------------------------
+// Stats (+ column checksums): per warp and column the max of the stored value image and the NULL count, into
+// s_wmax / s_wnull [NT / 32][n_cols]; four columns at a time, their loads in flight together.
+template <int NT, bool CKSUM>
+__device__ __forceinline__ void stats_pass(const Params &p, const uint32_t *tab, int64_t row0, uint32_t nrows, unsigned long long *s_wmax,
+                                           uint32_t *s_wnull, int tid, int lane, int warp) {
+  const int nc = p.n_cols;
   for (int c0 = 0; c0 < nc; c0 += 4) {
     unsigned long long mx[4] = {0, 0, 0, 0}, sum[4] = {0, 0, 0, 0};
     uint32_t nn[4] = {0, 0, 0, 0};
@@ -141,7 +127,7 @@ __global__ void __launch_bounds__(kThreads) obgpu_encode_blocks_kernel(const __g
 #pragma unroll
       for (int j = 0; j < 4; ++j) len_crc[j] = crc_word(tab, 0u, (uint32_t)p.col[min(c0 + j, nc - 1)].datum_len);
     }
-    for (uint32_t r = (uint32_t)tid; r < nrows; r += kThreads) {
+    for (uint32_t r = (uint32_t)tid; r < nrows; r += NT) {
       unsigned long long x[4];
       uint32_t nlb[4];
 #pragma unroll
@@ -192,6 +178,134 @@ __global__ void __launch_bounds__(kThreads) obgpu_encode_blocks_kernel(const __g
       }
     }
   }
+}
+
+// x (w <= 64 bits) at block bit address b of the zeroed shared-memory image: at most three shared atomicOr
+__device__ __forceinline__ void or_bits(uint32_t *img32, uint32_t b, uint32_t w, unsigned long long x) {
+  const uint32_t sh = b & 31u;
+  const unsigned long long xm = w >= 64u ? x : (x & ((1ull << w) - 1ull));
+  uint32_t *q = img32 + (b >> 5);
+  atomicOr(q, (uint32_t)(xm << sh));
+  if (sh + w > 32u) atomicOr(q + 1, (uint32_t)(xm >> (32u - sh)));
+  if (sh + w > 64u) atomicOr(q + 2, (uint32_t)(xm >> (64u - sh)));
+}
+
+// Output offset (thread 0): decoupled look-back over the aligned sizes (flag word: bits 63..62 state -- 1 aggregate, 2 inclusive
+// prefix --, low 62 bits bytes). Tickets are handed out in scheduling order, so every predecessor is running or done.
+__device__ __forceinline__ long long look_back(const Params &p, int blk, uint32_t size, uint32_t slot, bool host) {
+  volatile unsigned long long *flags = p.flags;
+  unsigned long long excl = 0;
+  if (blk > 0) {
+    int j = blk - 1;
+    for (;;) {
+      unsigned long long f;
+      do { f = flags[j]; } while ((f >> 62) == 0ull);
+      excl += f & ((1ull << 62) - 1ull);
+      if ((f >> 62) == 2ull) break;
+      --j;
+    }
+  }
+  flags[blk] = (2ull << 62) | (excl + slot);
+  p.blk_off[blk] = (int64_t)excl;
+  p.blk_size[blk] = size;
+  if (blk == p.n_blocks - 1) p.totals[0] = excl + slot;
+  if (host) atomicAdd(p.totals + 1, 1ull);
+  return (long long)excl;
+}
+
+// Payload checksum, every thread's share: the raw CRC of an odd-word-stride chunk, shifted to its position by one carry-less
+// multiplication and XOR-reduced per warp into s_red[warp]. Call after the image is complete and a barrier.
+template <int NT>
+__device__ __forceinline__ void payload_crc_part(const Params &p, const uint32_t *img32, const uint32_t *tab, uint32_t size, uint32_t *s_red,
+                                                 int tid, int lane, int warp) {
+  const uint32_t len = size - kHeaderSize, W = len >> 2;
+  uint32_t lw = (W + NT - 1u) / NT;
+  lw |= 1u;   // odd word stride between the threads' chunks: bank-conflict free
+  const int padw = (int)(NT * lw) - (int)W;   // leading zero words of the conceptual message
+  const uint32_t *pay = img32 + kHeaderSize / 4u;
+  uint32_t crc = 0;
+  {
+    const int w0 = tid * (int)lw - padw;
+    for (int w = max(w0, 0); w < w0 + (int)lw; ++w) crc = crc_word(tab, crc, pay[w]);
+  }
+  if (crc != 0) crc = gf2_mulmod(crc, p.xpow32[(uint32_t)(NT - 1 - tid) * lw]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) crc ^= __shfl_xor_sync(0xffffffffu, crc, o);
+  if (lane == 0) s_red[warp] = crc;
+}
+
+// Thread 0, after the barrier behind payload_crc_part: the payload crc's tail bytes, ObMicroBlockHeader
+// (ob_micro_block_header.h:95-153) + its 16-bit checksum (ob_micro_block_header.cpp:193-233), then ONE bulk copy of the slot.
+template <int NW>
+__device__ __forceinline__ void finish_block(const Params &p, uint8_t *smem, const uint32_t *tab, const uint32_t *s_red, uint32_t size,
+                                             uint32_t slot, uint32_t nrows, uint32_t ext_bit, uint32_t original, long long off) {
+  uint32_t *img32 = reinterpret_cast<uint32_t *>(smem);
+  const int nc = p.n_cols;
+  const uint32_t len = size - kHeaderSize;
+  uint32_t crc = 0;
+  for (int w = 0; w < NW; ++w) crc ^= s_red[w];
+  for (uint32_t k = len & ~3u; k < len; ++k) crc = crc_byte(tab, crc, smem[kHeaderSize + k]);
+  const uint32_t ncu = (uint32_t)nc, rk = (uint32_t)p.rowkey_cnt, flag16 = 1u << 2;   // all_lob_in_row_
+  const uint32_t opt = (ext_bit & 7u) << 3;                                            // row_index_byte 0, no var column
+  const uint32_t row_data_off = size;                                                  // meta end == block end
+  const uint16_t magic = (uint16_t)obf::MICRO_BLOCK_HEADER_MAGIC, version = (uint16_t)obf::MICRO_BLOCK_HEADER_VERSION;
+  uint32_t cs = 0;
+  auto f32 = [&](uint32_t x) { cs ^= (x & 0xffffu) ^ (x >> 16); };
+  cs ^= magic;
+  cs ^= version;
+  cs ^= (uint32_t)obf::ENCODING_ROW_STORE;
+  cs ^= opt;
+  f32(ncu); f32(rk); f32(flag16 & 1u); f32(0u /*opt2_: var column count*/);
+  f32(kHeaderSize); f32(nrows); f32(row_data_off); f32(original);
+  f32(len); f32(len); f32(crc);   // 64-bit fields with a zero high half fold like 32-bit ones
+  cs &= 0xffffu;
+  img32[0] = (uint32_t)magic | ((uint32_t)version << 16);
+  img32[1] = kHeaderSize;
+  img32[2] = cs | (ncu << 16);
+  img32[3] = rk | (flag16 << 16);
+  img32[4] = nrows;
+  img32[5] = (uint32_t)obf::ENCODING_ROW_STORE | (opt << 8);   // row_store_type_, opt_, opt2_ = 0
+  img32[6] = row_data_off;
+  img32[7] = original;
+  img32[8] = 0u; img32[9] = 0u;                 // max_merged_trans_version_
+  img32[10] = len;                              // data_length_
+  img32[11] = len;                              // data_zlength_
+  img32[12] = crc; img32[13] = 0u;              // data_checksum_
+  img32[14] = 0u; img32[15] = 0u;               // column_checksums_ptr_
+  // the other threads made their shared-memory writes visible to the async proxy before the barrier above
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  uint8_t *dst = p.image + off;
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(smem)), "r"(slot) : "memory");
+  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+}
+
+template <bool CKSUM>
+__global__ void __launch_bounds__(kThreads) obgpu_encode_blocks_kernel(const __grid_constant__ Params p) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  uint32_t *img32 = reinterpret_cast<uint32_t *>(smem);                 // block image, p.slot_cap bytes
+  uint32_t *tab = reinterpret_cast<uint32_t *>(smem + p.slot_cap);      // 4 x 256 crc tables
+  // per column scratch behind the tables: [kWarps][n_cols] max, [kWarps][n_cols] NULL count, [n_cols] layout
+  unsigned long long *s_wmax = reinterpret_cast<unsigned long long *>(smem + p.slot_cap + 4096u);
+  uint32_t *s_wnull = reinterpret_cast<uint32_t *>(s_wmax + kWarps * p.n_cols);
+  ColLayout *s_lay = reinterpret_cast<ColLayout *>(s_wnull + kWarps * p.n_cols);
+  __shared__ uint32_t s_red[kWarps];
+  __shared__ int s_blk;
+  __shared__ uint32_t s_size, s_original, s_ext_bit, s_host;
+  __shared__ long long s_off;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+
+  if (tid == 0) s_blk = atomicAdd(p.ticket, 1);
+  // zero image (cells are OR-ed in; padding up to the aligned slot must be zero): before anything else, under the ticket's round trip
+  for (uint32_t i = (uint32_t)tid; i < p.slot_cap / 16u; i += kThreads) reinterpret_cast<uint4 *>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
+  build_crc_tables<kThreads>(tab, tid);
+  const int blk = s_blk;
+  const int64_t row0 = (int64_t)blk * p.rows_per_block;
+  const uint32_t nrows = (uint32_t)min(p.rows_per_block, p.total_rows - row0);
+  const int nc = p.n_cols;
+  __syncthreads();
+
+  stats_pass<kThreads, CKSUM>(p, tab, row0, nrows, s_wmax, s_wnull, tid, lane, warp);
   __syncthreads();
 
   // ---- plan: warp 0, one lane per column (two rounds for more than 32 columns) -------------------------------------------
@@ -257,28 +371,7 @@ __global__ void __launch_bounds__(kThreads) obgpu_encode_blocks_kernel(const __g
   __syncthreads();
   const uint32_t size = s_size;
   const uint32_t slot = (size + p.align - 1u) & ~(p.align - 1u);
-  if (tid == 0) {
-    // ---- output offset: decoupled look-back over the aligned sizes (flag word: bits 63..62 state -- 1 aggregate, 2 inclusive
-    // prefix --, low 62 bits bytes). Tickets are handed out in scheduling order, so every predecessor is running or done.
-    volatile unsigned long long *flags = p.flags;
-    unsigned long long excl = 0;
-    if (blk > 0) {
-      int j = blk - 1;
-      for (;;) {
-        unsigned long long f;
-        do { f = flags[j]; } while ((f >> 62) == 0ull);
-        excl += f & ((1ull << 62) - 1ull);
-        if ((f >> 62) == 2ull) break;
-        --j;
-      }
-    }
-    flags[blk] = (2ull << 62) | (excl + slot);
-    s_off = (long long)excl;
-    p.blk_off[blk] = (int64_t)excl;
-    p.blk_size[blk] = size;
-    if (blk == p.n_blocks - 1) p.totals[0] = excl + slot;
-    if (s_host) atomicAdd(p.totals + 1, 1ull);
-  }
+  if (tid == 0) s_off = look_back(p, blk, size, slot, s_host != 0);
 
   if (size != 0) {
     // ---- pack ------------------------------------------------------------------------------------------------------------
@@ -307,77 +400,16 @@ __global__ void __launch_bounds__(kThreads) obgpu_encode_blocks_kernel(const __g
         const unsigned long long x = (unsigned long long)v[r] & cs.store_mask;
         // bit-packed cells: size bits each behind the ext bits; byte-packed cells: 8 * size bits each behind the bit area
         const uint32_t w = l.bp ? l.size : 8u * l.size;
-        const uint32_t b = (l.bp ? val0 : (l.store_off + l.bits_size) * 8u) + r * w, sh = b & 31u;
-        const unsigned long long xm = w >= 64u ? x : (x & ((1ull << w) - 1ull));
-        uint32_t *q = img32 + (b >> 5);
-        atomicOr(q, (uint32_t)(xm << sh));
-        if (sh + w > 32u) atomicOr(q + 1, (uint32_t)(xm >> (32u - sh)));
-        if (sh + w > 64u) atomicOr(q + 2, (uint32_t)(xm >> (64u - sh)));
+        or_bits(img32, (l.bp ? val0 : (l.store_off + l.bits_size) * 8u) + r * w, w, x);
       }
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // pack writes -> visible to the bulk copy issued by thread 0
     __syncthreads();
-    // ---- payload checksum ------------------------------------------------------------------------------------------------
-    const uint32_t len = size - kHeaderSize, W = len >> 2;
-    uint32_t lw = (W + kThreads - 1u) / kThreads;
-    lw |= 1u;   // odd word stride between the threads' chunks: bank-conflict free
-    const int padw = (int)(kThreads * lw) - (int)W;   // leading zero words of the conceptual message
-    const uint32_t *pay = img32 + kHeaderSize / 4u;
-    uint32_t crc = 0;
-    {
-      const int w0 = tid * (int)lw - padw;
-      for (int w = max(w0, 0); w < w0 + (int)lw; ++w) crc = crc_word(tab, crc, pay[w]);
-    }
-    if (crc != 0) crc = gf2_mulmod(crc, p.xpow32[(uint32_t)(kThreads - 1 - tid) * lw]);
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) crc ^= __shfl_xor_sync(0xffffffffu, crc, o);
-    if (lane == 0) s_red[warp] = crc;
+    payload_crc_part<kThreads>(p, img32, tab, size, s_red, tid, lane, warp);
   }
   __syncthreads();
 
-  if (tid == 0) {
-    if (size != 0) {
-      const uint32_t len = size - kHeaderSize;
-      uint32_t crc = 0;
-      for (int w = 0; w < kWarps; ++w) crc ^= s_red[w];
-      for (uint32_t k = len & ~3u; k < len; ++k) crc = crc_byte(tab, crc, smem[kHeaderSize + k]);
-      // ---- ObMicroBlockHeader (ob_micro_block_header.h:95-153) + its 16-bit checksum (ob_micro_block_header.cpp:193-233)
-      const uint32_t ncu = (uint32_t)nc, rk = (uint32_t)p.rowkey_cnt, flag16 = 1u << 2;   // all_lob_in_row_
-      const uint32_t opt = (s_ext_bit & 7u) << 3;                                          // row_index_byte 0, no var column
-      const uint32_t row_data_off = size;                                                  // meta end == block end
-      const uint32_t original = s_original;
-      const uint16_t magic = (uint16_t)obf::MICRO_BLOCK_HEADER_MAGIC, version = (uint16_t)obf::MICRO_BLOCK_HEADER_VERSION;
-      uint32_t cs = 0;
-      auto f32 = [&](uint32_t x) { cs ^= (x & 0xffffu) ^ (x >> 16); };
-      cs ^= magic;
-      cs ^= version;
-      cs ^= (uint32_t)obf::ENCODING_ROW_STORE;
-      cs ^= opt;
-      f32(ncu); f32(rk); f32(flag16 & 1u); f32(0u /*opt2_: var column count*/);
-      f32(kHeaderSize); f32(nrows); f32(row_data_off); f32(original);
-      f32(len); f32(len); f32(crc);   // 64-bit fields with a zero high half fold like 32-bit ones
-      cs &= 0xffffu;
-      img32[0] = (uint32_t)magic | ((uint32_t)version << 16);
-      img32[1] = kHeaderSize;
-      img32[2] = cs | (ncu << 16);
-      img32[3] = rk | (flag16 << 16);
-      img32[4] = nrows;
-      img32[5] = (uint32_t)obf::ENCODING_ROW_STORE | (opt << 8);   // row_store_type_, opt_, opt2_ = 0
-      img32[6] = row_data_off;
-      img32[7] = original;
-      img32[8] = 0u; img32[9] = 0u;                 // max_merged_trans_version_
-      img32[10] = len;                              // data_length_
-      img32[11] = len;                              // data_zlength_
-      img32[12] = crc; img32[13] = 0u;              // data_checksum_
-      img32[14] = 0u; img32[15] = 0u;               // column_checksums_ptr_
-      // the other threads made their shared-memory writes visible to the async proxy before the barrier above
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      uint8_t *dst = p.image + s_off;
-      asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(smem)), "r"(slot) : "memory");
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-      asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    }
-  }
+  if (tid == 0 && size != 0) finish_block<kWarps>(p, smem, tab, s_red, size, slot, nrows, s_ext_bit, s_original, s_off);
 }
 
 // Column checksums alone (ObMicroBlockChecksumHelper::cal_column_checksum over plain columns).
@@ -450,8 +482,12 @@ static const uint32_t *enc_xpow_table(obgpu_ctx *ctx) {
   std::lock_guard<std::mutex> g(mu);
   auto it = tables.find(ctx->device);
   if (it != tables.end()) return it->second;
-  const size_t lw_cap = (size_t)((ctx->max_smem_optin / 4 + enc::kThreads - 1) / enc::kThreads) | 1;
-  const size_t n_pow = (size_t)(enc::kThreads - 1) * lw_cap + 1;
+  // the RAW kernel's 128 threads and the codec kernel's 256 (encode_codecs.cuh) index it as (threads - 1 - tid) * chunk words
+  size_t n_pow = 1;
+  for (const size_t nt : {(size_t)enc::kThreads, (size_t)2 * enc::kThreads}) {
+    const size_t lw_cap = (size_t)((ctx->max_smem_optin / 4 + nt - 1) / nt) | 1;
+    n_pow = std::max(n_pow, (nt - 1) * lw_cap + 1);
+  }
   std::vector<uint32_t> xpow(n_pow);
   uint32_t b = 0x80000000u;
   for (size_t k = 0; k < n_pow; ++k) {
@@ -476,29 +512,27 @@ static int enc_fill_cols(enc::Params &p, const obgpu_encode_col *cols, int32_t n
     s.obj_type = (uint8_t)cols[c].obj_type;
     s.byte_only = cols[c].byte_packing_only ? 1 : 0;
     s.datum_len = (uint8_t)obf::datum_len_of((uint8_t)cols[c].obj_type);
+    s.sc = (uint8_t)sc;
+    s.ts = (uint8_t)obf::type_store_size((uint8_t)cols[c].obj_type);
   }
   p.n_cols = n_cols;
   return OBGPU_SUCCESS;
 }
 
-extern "C" {
-
-int obgpu_encode_columns(obgpu_ctx *ctx, const obgpu_encode_col *cols, int32_t n_cols, int32_t rowkey_col_cnt, int64_t total_rows,
-                         int64_t rows_per_block, int32_t align, obgpu_encoded **out) {
-  if (!ctx || !cols || !out || n_cols <= 0 || n_cols > enc::kMaxCols || rowkey_col_cnt < 0 || rowkey_col_cnt > n_cols || total_rows <= 0 ||
+// Checks the call's shape, fills p.col and allocates the handle's arena (flags, offsets, sizes, image of n_blocks slots) on the
+// context's stream; the caller sets the encodings and launches.
+static int enc_prepare(obgpu_ctx *ctx, const obgpu_encode_col *cols, int32_t n_cols, int32_t rowkey_col_cnt, int64_t total_rows,
+                       int64_t rows_per_block, int32_t align, enc::Params &p, int64_t &n_blocks64) {
+  if (!ctx || !cols || n_cols <= 0 || n_cols > enc::kMaxCols || rowkey_col_cnt < 0 || rowkey_col_cnt > n_cols || total_rows <= 0 ||
       rows_per_block <= 0 || rows_per_block > (1 << 22) || align < 16 || align > 4096 || (align & (align - 1)) != 0)
     return OBGPU_INVALID_ARGUMENT;
-  const int64_t n_blocks64 = (total_rows + rows_per_block - 1) / rows_per_block;
+  n_blocks64 = (total_rows + rows_per_block - 1) / rows_per_block;
   if (n_blocks64 > 0x7fffffff) return OBGPU_NOT_SUPPORTED;
-  enc::Params p{};
-  int rc = enc_fill_cols(p, cols, n_cols);
-  if (rc != OBGPU_SUCCESS) return rc;
-  cudaSetDevice(ctx->device);
-  // the largest block: every column 8 bytes wide + one ext bit per cell
-  const int64_t bound = (int64_t)enc::kHeaderSize + 16 * n_cols + (int64_t)n_cols * (rows_per_block * 8 + (rows_per_block + 7) / 8 + 1);
-  const int64_t slot_cap = (bound + align - 1) / align * align;
-  const size_t smem = (size_t)slot_cap + 4096 + (size_t)n_cols * (enc::kWarps * 12 + sizeof(enc::ColLayout)) + 16;
-  if ((int64_t)smem > (int64_t)ctx->max_smem_optin - 8192) return OBGPU_NOT_SUPPORTED;   // block image does not fit one CTA's shared memory
+  return enc_fill_cols(p, cols, n_cols);
+}
+
+static int enc_alloc(obgpu_ctx *ctx, enc::Params &p, int32_t n_cols, int32_t rowkey_col_cnt, int64_t total_rows, int64_t rows_per_block,
+                     int32_t align, int64_t n_blocks64, int64_t slot_cap, obgpu_encoded **out) {
   const uint32_t lw_max = (uint32_t)(((slot_cap / 4 + enc::kThreads - 1) / enc::kThreads) | 1);
   const uint32_t *d_xpow = enc_xpow_table(ctx);
   if (!d_xpow) return OBGPU_ALLOCATE_MEMORY_FAILED;
@@ -539,7 +573,23 @@ int obgpu_encode_columns(obgpu_ctx *ctx, const obgpu_encode_col *cols, int32_t n
   p.totals = e->d_totals;
   p.ticket = (int32_t *)(a + o_ctl + 128);
   p.xpow32 = d_xpow;
-  err = cudaFuncSetAttribute(enc::obgpu_encode_blocks_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  *out = e;
+  return OBGPU_SUCCESS;
+}
+
+// every column RAW: obgpu_encode_blocks_kernel
+static int enc_launch_raw(obgpu_ctx *ctx, enc::Params &p, int32_t n_cols, int32_t rowkey_col_cnt, int64_t total_rows, int64_t rows_per_block,
+                          int32_t align, int64_t n_blocks64, obgpu_encoded **out) {
+  // the largest block: every column 8 bytes wide + one ext bit per cell
+  const int64_t bound = (int64_t)enc::kHeaderSize + 16 * n_cols + (int64_t)n_cols * (rows_per_block * 8 + (rows_per_block + 7) / 8 + 1);
+  const int64_t slot_cap = (bound + align - 1) / align * align;
+  const size_t smem = (size_t)slot_cap + 4096 + (size_t)n_cols * (enc::kWarps * 12 + sizeof(enc::ColLayout)) + 16;
+  if ((int64_t)smem > (int64_t)ctx->max_smem_optin - 8192) return OBGPU_NOT_SUPPORTED;   // block image does not fit one CTA's shared memory
+  cudaSetDevice(ctx->device);
+  obgpu_encoded *e = nullptr;
+  int rc = enc_alloc(ctx, p, n_cols, rowkey_col_cnt, total_rows, rows_per_block, align, n_blocks64, slot_cap, &e);
+  if (rc != OBGPU_SUCCESS) return rc;
+  cudaError_t err = cudaFuncSetAttribute(enc::obgpu_encode_blocks_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) { ctx->err = cudaGetErrorString(err); obgpu_encoded_free(e); return OBGPU_ERR_SYS; }
   enc::obgpu_encode_blocks_kernel<true><<<(unsigned)e->n_blocks, enc::kThreads, smem, ctx->stream>>>(p);
   ctx->launches++;
@@ -547,6 +597,13 @@ int obgpu_encode_columns(obgpu_ctx *ctx, const obgpu_encode_col *cols, int32_t n
   if (err != cudaSuccess) { ctx->err = cudaGetErrorString(err); obgpu_encoded_free(e); return OBGPU_ERR_SYS; }
   *out = e;
   return OBGPU_SUCCESS;
+}
+
+extern "C" {
+
+int obgpu_encode_columns(obgpu_ctx *ctx, const obgpu_encode_col *cols, int32_t n_cols, int32_t rowkey_col_cnt, int64_t total_rows,
+                         int64_t rows_per_block, int32_t align, obgpu_encoded **out) {
+  return obgpu_encode_columns_with(ctx, cols, nullptr, n_cols, rowkey_col_cnt, total_rows, rows_per_block, align, out);
 }
 
 int obgpu_encoded_get_info(obgpu_encoded *e, obgpu_encoded_info *info) {
@@ -636,6 +693,11 @@ int obgpu_column_checksums(obgpu_ctx *ctx, const obgpu_encode_col *cols, int32_t
 
 int obgpu_merge_result_encode(obgpu_merge_result *res, const int32_t *result_cols, const int32_t *obj_types, int32_t n_cols,
                               int32_t rowkey_col_cnt, int64_t rows_per_block, int32_t align, obgpu_encoded **out) {
+  return obgpu_merge_result_encode_with(res, result_cols, obj_types, nullptr, n_cols, rowkey_col_cnt, rows_per_block, align, out);
+}
+
+int obgpu_merge_result_encode_with(obgpu_merge_result *res, const int32_t *result_cols, const int32_t *obj_types, const int32_t *encodings,
+                                   int32_t n_cols, int32_t rowkey_col_cnt, int64_t rows_per_block, int32_t align, obgpu_encoded **out) {
   if (!res || !result_cols || !obj_types || n_cols <= 0 || n_cols > enc::kMaxCols || !out) return OBGPU_INVALID_ARGUMENT;
   obgpu_merge_info info;
   int rc = obgpu_merge_result_info(res, &info);
@@ -660,7 +722,7 @@ int obgpu_merge_result_encode(obgpu_merge_result *res, const int32_t *result_col
       c.dev_null = res->out_null[(size_t)k];
     }
   }
-  return obgpu_encode_columns(res->ctx, cols.data(), n_cols, rowkey_col_cnt, info.out_rows, rows_per_block, align, out);
+  return obgpu_encode_columns_with(res->ctx, cols.data(), encodings, n_cols, rowkey_col_cnt, info.out_rows, rows_per_block, align, out);
 }
 
 }  // extern "C"

@@ -3659,6 +3659,7 @@ int obgpu_project_datums(obgpu_batch *batch, int32_t block, int32_t col, const i
 #include "merge_exchange.cuh"
 #include "merge_streamed.cuh"
 #include "encode_kernels.cuh"   // phase B: merged columns -> SSTable bytes + column checksums
+#include "encode_codecs.cuh"    // phase B with DICT / RLE / CONST / INTEGER_BASE_DIFF columns, or the codec chosen per micro-block
 
 // ---- host-buffer scan pipeline (include/obgpu_pipeline.h) ------------------------------------------------
 #include "host_pipeline.h"

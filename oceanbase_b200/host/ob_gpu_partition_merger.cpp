@@ -125,9 +125,10 @@ int ObGpuPartitionMajorMerger::write_column_groups(const std::vector<ObGpuColumn
   std::vector<obgpu_encoded *> enc(groups.size(), nullptr);
   for (size_t g = 0; OB_SUCCESS == ret && g < groups.size(); ++g) {
     const ObGpuColumnGroup &cg = groups[g];
-    if (cg.cols_.empty() || cg.cols_.size() != cg.obj_types_.size()) ret = OB_INVALID_ARGUMENT;
-    else ret = obgpu_merge_result_encode(result_, cg.cols_.data(), cg.obj_types_.data(), (int32_t)cg.cols_.size(), cg.rowkey_col_cnt_,
-                                         rows_per_block, align, &enc[g]);
+    if (cg.cols_.empty() || cg.cols_.size() != cg.obj_types_.size() || (!cg.encodings_.empty() && cg.encodings_.size() != cg.cols_.size()))
+      ret = OB_INVALID_ARGUMENT;
+    else ret = obgpu_merge_result_encode_with(result_, cg.cols_.data(), cg.obj_types_.data(), cg.encodings_.empty() ? nullptr : cg.encodings_.data(),
+                                              (int32_t)cg.cols_.size(), cg.rowkey_col_cnt_, rows_per_block, align, &enc[g]);
   }
   for (size_t g = 0; OB_SUCCESS == ret && g < groups.size(); ++g) {
     const ObGpuColumnGroup &cg = groups[g];
@@ -144,8 +145,9 @@ int ObGpuPartitionMajorMerger::write_column_groups(const std::vector<ObGpuColumn
     ret = obgpu_encoded_fetch(enc[g], o.image_.data(), info.image_size, o.offsets_.data(), o.sizes_.data(), info.n_blocks);
     if (OB_SUCCESS == ret) ret = obgpu_encoded_column_checksums(enc[g], o.column_checksums_.data());
     if (OB_SUCCESS == ret && info.n_host_blocks > 0) {
-      // the blocks the device left out (ObRawEncoder stores a NULL-dominated column as var-length cells): their rows come
-      // back as rows and go through the host writer; the image is laid out again with them in place
+      // the blocks the device left out (ObRawEncoder stores a NULL-dominated column as var-length cells, or a forced codec the
+      // block's data does not take): their rows come back as rows and go through the host writer with the same encodings; the
+      // image is laid out again with them in place
       std::vector<uint8_t> image;
       std::vector<int64_t> offsets((size_t)info.n_blocks);
       std::vector<int64_t> vals;
@@ -166,7 +168,7 @@ int ObGpuPartitionMajorMerger::write_column_groups(const std::vector<ObGpuColumn
                                            cg.cols_[c] >= 0 ? nulls.data() + c * (size_t)n : nullptr);
             in[c] = obgpu_col_input{};
             in[c].obj_type = cg.obj_types_[c];
-            in[c].encoding = OBGPU_ENC_RAW;
+            in[c].encoding = cg.encodings_.empty() ? OBGPU_ENC_RAW : cg.encodings_[c];
             in[c].i64 = vals.data() + c * (size_t)n;
             in[c].is_null = nulls.data() + c * (size_t)n;
           }

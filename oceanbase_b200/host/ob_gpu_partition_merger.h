@@ -56,6 +56,8 @@ struct ObGpuColumnGroup {
   std::vector<int32_t> cols_;
   std::vector<int32_t> obj_types_;   // OBGPU_OBJ_* of every column (integer classes)
   int32_t rowkey_col_cnt_ = 0;       // > 0 for the group that carries the rowkey (all-column / rowkey group)
+  // OBGPU_ENC_RAW / _DICT / _RLE / _CONST / _INTEGER_BASE_DIFF / _AUTO of every column; empty: every column RAW
+  std::vector<int32_t> encodings_;
 };
 
 // What the writer of one column group produced: the micro-blocks of its SSTable + the column checksums of its rows.
@@ -64,7 +66,7 @@ struct ObGpuEncodedColumnGroup {
   std::vector<int64_t> offsets_, sizes_;
   std::vector<int64_t> column_checksums_;
   int64_t row_count_ = 0;
-  int32_t host_encoded_blocks_ = 0;  // blocks the device left to the host writer (a NULL-dominated column stored as var cells)
+  int32_t host_encoded_blocks_ = 0;  // blocks the device left to the host writer (var-stored RAW cells, a codec refused for the block)
 };
 
 class ObGpuPartitionMajorMerger {
@@ -87,8 +89,9 @@ public:
   // Column-oriented merge, writer side (ObCOMergeLogReplayer::replay_merge_log -> ObCOMergeWriter::replay_mergelog ->
   // ObWriteHelper::project / append, column_store/ob_column_oriented_merger.cpp:722-745, ob_co_merge_writer.cpp:67-117,345):
   // the merged stream -- produced once by merge_partition -- is replayed into the writer of every column group. Here a
-  // writer is the device encoder (obgpu_merge_result_encode): the rows never leave the device as rows, each group comes back
-  // as reference-format micro-blocks (every column RAW) + its column checksums. rows_per_block cuts the blocks.
+  // writer is the device encoder (obgpu_merge_result_encode_with): the rows never leave the device as rows, each group comes
+  // back as reference-format micro-blocks (the group's encodings_, RAW when empty) + its column checksums. rows_per_block cuts
+  // the blocks; a block the device leaves out is encoded by the host writer with the same encodings and spliced in.
   int write_column_groups(const std::vector<ObGpuColumnGroup> &groups, int64_t rows_per_block, int32_t align,
                           std::vector<ObGpuEncodedColumnGroup> &out);
   void reset();

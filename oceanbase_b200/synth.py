@@ -319,3 +319,43 @@ def filter_columns(expr):
     for c in expr.children:
         out += filter_columns(c)
     return sorted(set(out))
+
+
+# ---- device encoder shapes (tools/bench_encode.py, tests/test_gpu_device_encoder_codecs.py) ------------------------------------
+ENCODE_SHAPES = ("cfg5", "lineitem", "eventlog")
+
+
+def make_encode_columns(shape: str, n: int, seed: int = 5, device="cuda"):
+    """Integer columns for the device encoder, generated with torch on `device` from `seed`, rowkey first:
+    [(OBJ_* type, int64 values, uint8 NULL bytes or None)].
+      cfg5     : key = 3 i + 1e9 + 7; 33-bit; 63-bit signed; 13-bit with 5 % NULLs
+      lineitem : sorted orderkey with up to 4 lines an order; quantity 1..50; discount 0..10; tax 0..8; DATE over 2 526 days;
+                 price; a 3-value status in runs of 50 rows
+      eventlog : DATETIME in microseconds, increasing; 8 tenant ids of up to 900 123; HTTP status 97 % 200; user id in a 10^6
+                 range above 10^12; 20-bit latency"""
+    import torch
+    g = torch.Generator(device=device).manual_seed(seed)
+
+    def rnd(lo, hi):
+        return torch.randint(lo, hi, (n,), device=device, dtype=torch.int64, generator=g)
+
+    i = torch.arange(n, device=device, dtype=torch.int64)
+    if shape == "cfg5":
+        nl = (torch.rand((n,), device=device, generator=g) < 0.05).to(torch.uint8)
+        return [(capi.OBJ_INT, i * 3 + 1_000_000_007, None), (capi.OBJ_INT, rnd(0, 1 << 33), None),
+                (capi.OBJ_INT, rnd(-(1 << 62), 1 << 62), None), (capi.OBJ_INT, rnd(0, 1 << 13), nl)]
+    if shape == "lineitem":
+        orderkey = torch.cumsum((torch.rand((n,), device=device, generator=g) < 0.25).to(torch.int64), 0) * 32 + 1   # ~4 lines an order
+        runs = torch.randint(0, 3, ((n + 49) // 50,), device=device, dtype=torch.int64, generator=g)
+        status = torch.tensor([70, 79, 80], device=device, dtype=torch.int64)[runs].repeat_interleave(50)[:n]
+        return [(capi.OBJ_INT, orderkey, None), (capi.OBJ_INT, rnd(1, 51), None), (capi.OBJ_INT, rnd(0, 11), None),
+                (capi.OBJ_INT, rnd(0, 9), None), (capi.OBJ_DATE, rnd(8035, 8035 + 2526), None), (capi.OBJ_INT, rnd(90_000, 10_500_000), None),
+                (capi.OBJ_INT, status, None)]
+    if shape == "eventlog":
+        ts = 1_700_000_000_000_000 + torch.cumsum(rnd(1, 2000), 0)
+        tenants = torch.randint(1, 900_124, (8,), device=device, dtype=torch.int64, generator=g)
+        other = torch.tensor([302, 404, 500], device=device, dtype=torch.int64)
+        status = torch.where(torch.rand((n,), device=device, generator=g) < 0.97, torch.full_like(i, 200), other[rnd(0, 3)])
+        return [(capi.OBJ_DATETIME, ts, None), (capi.OBJ_INT, tenants[rnd(0, 8)], None), (capi.OBJ_INT, status, None),
+                (capi.OBJ_INT, 10**12 + rnd(0, 10**6), None), (capi.OBJ_INT, rnd(0, 1 << 20), None)]
+    raise ValueError(f"shape {shape!r}: one of {ENCODE_SHAPES}")
